@@ -45,6 +45,7 @@ WORKLOADS = {
     "embedding_1e6x1e3": ([("P", (1_000_000, 1_000))], 1, None),
 }
 MODES = {"sum": 1, "async": 0, "mean": 2}
+DUMP_BYTES = 48 << 20       # --dump-outputs: all arrays together stay below 64 MB
 
 
 def parse():
@@ -90,7 +91,15 @@ def parse():
     p.add_argument("--cpu-sample-elems", type=int, default=100_000_000,
                    help="CPU arms: parameters per step -- the SAME absolute sample at every "
                         "N, pushed / pulled by N workers")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR", default=None,
+                   help="after the timed steps, write the parameters worker 0 pulled in the "
+                        "last one as DIR/<variable>.npy (float32; a variable too large for "
+                        "its share of %d MiB is sampled at fixed, seeded positions)"
+                        % (DUMP_BYTES >> 20))
+    args = p.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        p.error("--dump-outputs writes what the CUDA path computed: use it with --impl b200")
+    return args
 
 
 def n_params(workload):
@@ -542,6 +551,31 @@ def verify_cluster(cl, mode_name, wire_name, dist, host=False, samples=1_000_000
     return out
 
 
+def dump_index(numel, n_vars):
+    """Positions of a variable that --dump-outputs writes: all of them when the
+    variable fits its share of DUMP_BYTES, else a sorted sample drawn with a
+    fixed seed -- the same positions on every run and in every build."""
+    import numpy as np
+    cap = DUMP_BYTES // 4 // max(1, n_vars)
+    if numel <= cap:
+        return None
+    return np.sort(np.random.default_rng(0).choice(numel, cap, replace=False))
+
+
+def dump_outputs(worker, out_dir):
+    """Write what the timed round handed `worker` in its last step: every
+    variable's pulled parameters, as float32 <out_dir>/<name>.npy."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in worker.params.items():
+        flat = t.reshape(-1)
+        idx = dump_index(flat.numel(), len(worker.params))
+        if idx is not None:
+            flat = flat[torch.from_numpy(idx).to(flat.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), flat.float().cpu().numpy())
+
+
 def resolve_path(args, world, psx, local_rank):
     if args.path in ("staged", "nvls"):
         return args.path
@@ -657,6 +691,8 @@ def run_b200(args):
         sampler.start()
     timer = KernelTimer()
     ms_step, launches = timed(steps, timer=timer)
+    if args.dump_outputs and cl.worker is not None and cl.worker.index == 0:
+        dump_outputs(cl.worker, args.dump_outputs)
     bytes_step = W * n_full * 2 * esz           # W * N * (s_g + s_p)
     value = bytes_step / (ms_step * 1e-3) / 1e9
     verified = None if args.no_verify else verify_cluster(cl, args.mode, args.wire, dist)

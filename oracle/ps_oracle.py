@@ -20,6 +20,7 @@ from __future__ import annotations
 import ctypes
 import os
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -230,10 +231,17 @@ _LIB = None
 
 def build_c(force=False):
     out_dir = os.path.join(HERE, "_build")
-    os.makedirs(out_dir, exist_ok=True)
     so = os.path.join(out_dir, "libps_oracle.so")
     src = os.path.join(HERE, "ps_oracle.c")
     if force or not os.path.exists(so) or os.path.getmtime(so) < os.path.getmtime(src):
+        try:
+            os.makedirs(out_dir, exist_ok=True)
+        except OSError:
+            pass
+        if not os.access(out_dir, os.W_OK):
+            # a read-only tree (e.g. a benchmark run from an installed checkout):
+            # build beside it, never into it
+            so = os.path.join(tempfile.mkdtemp(prefix="ps_oracle_"), "libps_oracle.so")
         subprocess.check_call(
             ["gcc", "-O2", "-std=c11", "-ffp-contract=off", "-fno-fast-math",
              "-fPIC", "-shared", src, "-o", so, "-lm", "-lpthread"])

@@ -160,6 +160,11 @@ def run_case(case, rounds, rank, world, device, dist):
     def fill(rnd, host=False):
         if wk is None:
             return
+        if host:
+            # the last round_host's H2D copies read the pinned gradients
+            # asynchronously (behind the other ranks' pushes); they are free
+            # again once the worker stream has passed them
+            ws.synchronize()
         for t in range(cl.layout.ps_tasks):
             n = wk.grad_flat[t].numel()
             if host:

@@ -36,7 +36,11 @@ def _launch(world, cases, rounds=3, timeout=1100, only=None):
     env = dict(os.environ, PYTHONUNBUFFERED="1", OMP_NUM_THREADS="4")
     p = subprocess.run(cmd, cwd=ROOT, env=env, stdout=subprocess.PIPE, stderr=subprocess.STDOUT,
                        text=True, timeout=timeout)
-    tail = "\n".join(p.stdout.splitlines()[-60:])
+    # the per-case verdicts and every rank's errors first: torchrun's own report of
+    # the failed children fills the end of the output
+    lines = p.stdout.splitlines()
+    verdicts = [l for l in lines if l.startswith(("CASE", "[rank", "MULTIRANK"))]
+    tail = "\n".join(verdicts[-60:] + ["..."] + lines[-20:])
     assert p.returncode == 0, "multirank parity failed (world %d, %s):\n%s" % (world, cases, tail)
     assert "MULTIRANK PARITY: all ok" in p.stdout, tail
     return p.stdout

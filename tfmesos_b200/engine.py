@@ -777,7 +777,10 @@ class TorchrunCluster(object):
         pushes, so it can only complete (and its pull / D2H start) when the slowest
         rank has reached it -- identical order makes that as early as possible, and
         the pushes are PCIe-paced (49 GB/s per rank), far below what incast into one
-        NVLink port would need to matter."""
+        NVLink port would need to matter.
+        Returns once the round is enqueued: ``staging.grad`` and ``staging.param``
+        belong to it until ``worker_stream`` has passed its end, so synchronise
+        that stream before rewriting the gradients or reading the parameters."""
         import torch
         assert self.worker is not None and not self.fused, \
             "round_host runs on worker ranks of a staged-path cluster"
