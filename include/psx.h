@@ -43,7 +43,7 @@
 extern "C" {
 #endif
 
-#define PSX_ABI_VERSION 10
+#define PSX_ABI_VERSION 11
 
 /* error codes */
 #define PSX_OK 0
@@ -53,9 +53,21 @@ extern "C" {
 #define PSX_ESTATE (-4)   /* call not valid in the object's current state     */
 #define PSX_EABI (-5)     /* handle blob from another ABI version             */
 
-/* optimizers (reference: mnist.py:55 / mnist_replica.py:147) */
+/* optimizers (reference: mnist.py:55 / mnist_replica.py:147; the others are
+ * TF 0.12's ApplyMomentum / ApplyAdagrad / ApplyRMSProp).  The shard layout
+ * depends on the optimizer, so a handle blob only opens in a build of the same ABI.
+ *   opt       hyper[4]                       PSX_M              PSX_V     initial M / V
+ *   SGD       {lr, -, -, -}                  -                  -
+ *   ADAM      {lr, beta1, beta2, epsilon}    m                  v         0 / 0
+ *   MOMENTUM  {lr, momentum, -, -}           accum              -         0
+ *   ADAGRAD   {lr, initial_accum, -, -}      accum              -         initial_accum (> 0)
+ *   RMSPROP   {lr, decay, momentum, eps}     ms (rms)           mom       1 / 0
+ * Only Adam keeps beta powers; the others advance global_step alone. */
 #define PSX_OPT_SGD 0
 #define PSX_OPT_ADAM 1
+#define PSX_OPT_MOMENTUM 2
+#define PSX_OPT_ADAGRAD 3
+#define PSX_OPT_RMSPROP 4
 
 /* update disciplines (SURVEY.md appendix A.4) */
 #define PSX_MODE_ASYNC_ORDERED 0 /* each slot applied on its own, slot order  */
@@ -94,9 +106,10 @@ int psx_enable_peer(int device, int peer);
 /* ------------------------------------------------------------------ PS side */
 
 /* Allocate one PS shard in HBM on `device`: a flat f32 bucket `var[nelem]`
- * (+ Adam `m`,`v`, stored beta powers, global_step) and `n_slots` gradient
- * landing slots of `wire_dtype`, plus the flag words the kernels synchronise
- * on.  hyper = {lr, beta1, beta2, epsilon}.
+ * (+ the optimizer's state arrays, stored beta powers, global_step) and `n_slots`
+ * gradient landing slots of `wire_dtype`, plus the flag words the kernels
+ * synchronise on.  hyper: see the optimizer table above; an unknown `opt` or an
+ * Adagrad initial accumulator <= 0 fails with PSX_EINVAL.
  * Replaces: variables + slot variables created on /job:ps/task:k by
  * replica_device_setter (mnist.py:43-46, mnist_replica.py:116-134) and
  * tf.get_variable under tf.device (matrix_factorization.py:21-28). */
@@ -116,7 +129,7 @@ int psx_get_values(uint64_t id, int which, float *host, uint64_t off, uint64_t n
 int psx_get_state(uint64_t id, float *b1p, float *b2p, int64_t *step, uint32_t *apply_seq);
 int psx_set_state(uint64_t id, float b1p, float b2p, int64_t step);
 
-/* Fused reduce(slots) + SGD/Adam + beta-power / global_step update over the
+/* Fused reduce(slots) + optimizer update + beta-power / global_step update over the
  * whole shard.  If wait_seq != 0 the stream first waits (cuStreamWaitValue32,
  * no SM is held) until every slot in [first_slot, first_slot+count) has been
  * pushed with seq >= wait_seq.  On completion the shard's apply_seq is
@@ -247,7 +260,7 @@ int psx_mailbox_set(uint64_t id, uint32_t value);
 
 /* ONE kernel on the PS GPU: gather the bound gradients straight from the
  * workers' HBM (peer loads), reduce in registers in slot order, apply
- * SGD/Adam to var/m/v in place, and scatter the new parameters into every
+ * the optimizer to var/m/v in place, and scatter the new parameters into every
  * bound parameter buffer (peer stores) -- push + sum + apply + pull with no
  * staging copy.  Waits like psx_apply. */
 int psx_round(uint64_t shard_id, int mode, int first_slot, int count, uint32_t wait_seq,
@@ -332,7 +345,7 @@ int psx_read_step_async(uint64_t client_id, int64_t *host_pinned, void *stream);
  * into this worker's landing slot and publishes `seq` like psx_push.
  * psx_apply_rows waits for the slots like psx_apply, merges rows pushed by
  * several workers in worker order (binary search, no float atomics: bit-
- * reproducible), divides by `count` for SYNC_MEAN, and applies SGD / Adam ONCE to
+ * reproducible), divides by `count` for SYNC_MEAN, and applies the optimizer ONCE to
  * every touched row -- untouched rows keep var, m and v; beta powers and
  * global_step advance once per call. */
 int psx_push_rows(uint64_t client_id, const int64_t *idx_dev, const void *rows_dev, uint64_t k,

@@ -2,8 +2,8 @@
 reference gets from ``tf.train.Supervisor(logdir=...)`` (TF checkpoints written
 by the chief, examples/mnist/mnist_replica.py:165-170).
 
-One safetensors file per process: every hosted stripe's ``var`` (+ Adam ``m``,
-``v``) as float32 tensors keyed ``<region>/ps<task>/stripe<j>``, and the scalars
+One safetensors file per process: every hosted stripe's ``var`` (+ the
+optimizer's state arrays ``m`` [, ``v``]) as float32 tensors keyed ``<region>/ps<task>/stripe<j>``, and the scalars
 (global_step, stored beta powers) in the metadata.  Restoring puts back exactly
 those bits, so a resumed run continues bit-identically (tests/test_gpu_checkpoint.py).
 """
@@ -14,7 +14,8 @@ from . import psx
 
 
 def _regions(ps):
-    return [("var", psx.VAR)] + ([("m", psx.M), ("v", psx.V)] if ps.shard.opt == psx.OPT_ADAM else [])
+    n_state = psx.OPT_STATE_ARRAYS[ps.shard.opt]
+    return [("var", psx.VAR), ("m", psx.M), ("v", psx.V)][:1 + n_state]
 
 
 def shard_file(path, rank=0, world=1):

@@ -119,14 +119,28 @@ struct HandleBlob {           // PSX_HANDLE_BYTES, shipped between processes
 };
 static_assert(sizeof(HandleBlob) == PSX_HANDLE_BYTES, "handle blob size");
 
+// f32 state arrays the optimizer keeps beside var (OptTraits::kState); -1: unknown id
+int state_arrays(int opt)
+{
+    switch (opt) {
+    case PSX_OPT_SGD: return OptTraits<PSX_OPT_SGD>::kState;
+    case PSX_OPT_ADAM: return OptTraits<PSX_OPT_ADAM>::kState;
+    case PSX_OPT_MOMENTUM: return OptTraits<PSX_OPT_MOMENTUM>::kState;
+    case PSX_OPT_ADAGRAD: return OptTraits<PSX_OPT_ADAGRAD>::kState;
+    case PSX_OPT_RMSPROP: return OptTraits<PSX_OPT_RMSPROP>::kState;
+    default: return -1;
+    }
+}
+
 struct Layout {
     uint64_t nelem = 0, nelem_pad = 0;
     int opt = 0, n_slots = 0, wire = 0;
     size_t wire_bytes() const { return wire == PSX_BF16 ? 2 : 4; }
+    int n_state() const { return state_arrays(opt); }
     size_t off_var() const { return kHeaderBytes; }
     size_t off_m() const { return off_var() + nelem_pad * 4; }
-    size_t off_v() const { return off_m() + (opt == PSX_OPT_ADAM ? nelem_pad * 4 : 0); }
-    size_t off_slots() const { return off_v() + (opt == PSX_OPT_ADAM ? nelem_pad * 4 : 0); }
+    size_t off_v() const { return off_m() + (n_state() >= 1 ? nelem_pad * 4 : 0); }
+    size_t off_slots() const { return off_v() + (n_state() >= 2 ? nelem_pad * 4 : 0); }
     size_t total() const { return off_slots() + (size_t)n_slots * nelem_pad * wire_bytes(); }
 };
 
@@ -365,14 +379,19 @@ int launch_apply(Shard *s, int mode, SRC src, int count, const PeerSet &peers, c
 {
     if (r.n == 0 && r.off == 0) r.n = s->lay.nelem_pad;
 #define PSX_AP(O, M) launch_apply_t<O, M, SCATTER, SRC>(s, src, count, peers, st, r)
+#define PSX_AP3(O)                                                                            \
+    if (mode == PSX_MODE_ASYNC_ORDERED) PSX_AP(O, PSX_MODE_ASYNC_ORDERED);                    \
+    else if (mode == PSX_MODE_SUM) PSX_AP(O, PSX_MODE_SUM);                                   \
+    else if (mode == PSX_MODE_SYNC_MEAN) PSX_AP(O, PSX_MODE_SYNC_MEAN);                       \
+    else return fail(PSX_EINVAL, "unknown optimizer/mode %d/%d", opt, mode)
     const int opt = s->lay.opt;
-    if (opt == PSX_OPT_SGD && mode == PSX_MODE_ASYNC_ORDERED) PSX_AP(PSX_OPT_SGD, PSX_MODE_ASYNC_ORDERED);
-    else if (opt == PSX_OPT_SGD && mode == PSX_MODE_SUM) PSX_AP(PSX_OPT_SGD, PSX_MODE_SUM);
-    else if (opt == PSX_OPT_SGD && mode == PSX_MODE_SYNC_MEAN) PSX_AP(PSX_OPT_SGD, PSX_MODE_SYNC_MEAN);
-    else if (opt == PSX_OPT_ADAM && mode == PSX_MODE_ASYNC_ORDERED) PSX_AP(PSX_OPT_ADAM, PSX_MODE_ASYNC_ORDERED);
-    else if (opt == PSX_OPT_ADAM && mode == PSX_MODE_SUM) PSX_AP(PSX_OPT_ADAM, PSX_MODE_SUM);
-    else if (opt == PSX_OPT_ADAM && mode == PSX_MODE_SYNC_MEAN) PSX_AP(PSX_OPT_ADAM, PSX_MODE_SYNC_MEAN);
+    if (opt == PSX_OPT_SGD) { PSX_AP3(PSX_OPT_SGD); }
+    else if (opt == PSX_OPT_ADAM) { PSX_AP3(PSX_OPT_ADAM); }
+    else if (opt == PSX_OPT_MOMENTUM) { PSX_AP3(PSX_OPT_MOMENTUM); }
+    else if (opt == PSX_OPT_ADAGRAD) { PSX_AP3(PSX_OPT_ADAGRAD); }
+    else if (opt == PSX_OPT_RMSPROP) { PSX_AP3(PSX_OPT_RMSPROP); }
     else return fail(PSX_EINVAL, "unknown optimizer/mode %d/%d", opt, mode);
+#undef PSX_AP3
 #undef PSX_AP
     LAUNCH_CHECK();
     return PSX_OK;
@@ -405,11 +424,17 @@ int launch_round_mc(Shard *s, int mode, const PeerSet &peers, cudaStream_t st, c
         (float4 *)(s->v() + r.off), s->mc_grad + r.off, s->mc_param + r.off, n4, peers,       \
         r.consume, r.divisor)
     const int opt = s->lay.opt;
-    if (opt == PSX_OPT_SGD && mode == PSX_MODE_SUM) PSX_MC(PSX_OPT_SGD, PSX_MODE_SUM);
-    else if (opt == PSX_OPT_SGD && mode == PSX_MODE_SYNC_MEAN) PSX_MC(PSX_OPT_SGD, PSX_MODE_SYNC_MEAN);
-    else if (opt == PSX_OPT_ADAM && mode == PSX_MODE_SUM) PSX_MC(PSX_OPT_ADAM, PSX_MODE_SUM);
-    else if (opt == PSX_OPT_ADAM && mode == PSX_MODE_SYNC_MEAN) PSX_MC(PSX_OPT_ADAM, PSX_MODE_SYNC_MEAN);
+#define PSX_MC2(O)                                                                            \
+    if (mode == PSX_MODE_SUM) PSX_MC(O, PSX_MODE_SUM);                                        \
+    else if (mode == PSX_MODE_SYNC_MEAN) PSX_MC(O, PSX_MODE_SYNC_MEAN);                       \
+    else return fail(PSX_EINVAL, "the NVLS round supports SUM / SYNC_MEAN (optimizer/mode %d/%d)", opt, mode)
+    if (opt == PSX_OPT_SGD) { PSX_MC2(PSX_OPT_SGD); }
+    else if (opt == PSX_OPT_ADAM) { PSX_MC2(PSX_OPT_ADAM); }
+    else if (opt == PSX_OPT_MOMENTUM) { PSX_MC2(PSX_OPT_MOMENTUM); }
+    else if (opt == PSX_OPT_ADAGRAD) { PSX_MC2(PSX_OPT_ADAGRAD); }
+    else if (opt == PSX_OPT_RMSPROP) { PSX_MC2(PSX_OPT_RMSPROP); }
     else return fail(PSX_EINVAL, "the NVLS round supports SUM / SYNC_MEAN (optimizer/mode %d/%d)", opt, mode);
+#undef PSX_MC2
 #undef PSX_MC
     LAUNCH_CHECK();
     return PSX_OK;
@@ -629,7 +654,9 @@ int psx_shard_create(int device, uint64_t nelem, int opt, const float *hyper, in
 {
     if (!out_id || !hyper) return fail(PSX_EINVAL, "null argument");
     if (nelem == 0) return fail(PSX_EINVAL, "empty shard");
-    if (opt != PSX_OPT_SGD && opt != PSX_OPT_ADAM) return fail(PSX_EINVAL, "unknown optimizer %d", opt);
+    if (state_arrays(opt) < 0) return fail(PSX_EINVAL, "unknown optimizer %d", opt);
+    if (opt == PSX_OPT_ADAGRAD && !(hyper[1] > 0.0f))
+        return fail(PSX_EINVAL, "Adagrad initial_accumulator_value must be > 0 (got %g)", (double)hyper[1]);
     if (n_slots < 0 || n_slots > PSX_MAX_SLOTS) return fail(PSX_EINVAL, "n_slots %d not in [0,%d]", n_slots, PSX_MAX_SLOTS);
     if (wire_dtype != PSX_F32 && wire_dtype != PSX_BF16) return fail(PSX_EINVAL, "unknown wire dtype %d", wire_dtype);
     PSX_DEVICE(device);
@@ -663,6 +690,16 @@ int psx_shard_create(int device, uint64_t nelem, int opt, const float *hyper, in
     h.b1p = hyper[1];  // powers start at beta (AdamOptimizer._create_slots)
     h.b2p = hyper[2];
     if (e == cudaSuccess) e = cudaMemcpy(p, &h, sizeof(h), cudaMemcpyHostToDevice);
+    // accumulators that do not start at zero: Adagrad's at initial_accumulator_value,
+    // RMSProp's ms at 1 (TF's `rms` slot initializer); padding included
+    const float m0 = opt == PSX_OPT_ADAGRAD ? hyper[1] : opt == PSX_OPT_RMSPROP ? 1.0f : 0.0f;
+    if (e == cudaSuccess && m0 != 0.0f) {
+        const size_t n4 = s->lay.nelem_pad / 4;
+        k_fill<<<grid_for(n4, kCopyThreads, s->sm_count, 8), kCopyThreads>>>((float4 *)s->m(), m0, n4);
+        e = cudaGetLastError();
+        if (e == cudaSuccess) e = cudaDeviceSynchronize();
+        if (e == cudaSuccess) g_launches.fetch_add(1, std::memory_order_relaxed);
+    }
     if (e != cudaSuccess) {
         cudaFree(p);
         delete s;
@@ -748,8 +785,8 @@ static int region_of(Shard *s, int which, char **base, int *dtype)
 {
     *dtype = PSX_F32;
     if (which == PSX_VAR) *base = (char *)s->var();
-    else if (which == PSX_M && s->lay.opt == PSX_OPT_ADAM) *base = (char *)s->m();
-    else if (which == PSX_V && s->lay.opt == PSX_OPT_ADAM) *base = (char *)s->v();
+    else if (which == PSX_M && s->lay.n_state() >= 1) *base = (char *)s->m();
+    else if (which == PSX_V && s->lay.n_state() >= 2) *base = (char *)s->v();
     else if (which >= PSX_SLOT0 && which < PSX_SLOT0 + s->lay.n_slots) {
         *base = s->slot(which - PSX_SLOT0);
         *dtype = s->lay.wire;
@@ -1436,10 +1473,14 @@ int psx_apply_rows(uint64_t id, int mode, int first_slot, int count, uint64_t ro
 #define PSX_AR(O, M, W) k_apply_rows<O, M, W><<<grid, 256, 0, st>>>(s->hdr(), s->var(), s->m(), s->v(), s->slot(0), stride, first_slot, count, (size_t)row_len, n_rows, peers)
 #define PSX_AR2(O, M) do { if (s->lay.wire == PSX_F32) PSX_AR(O, M, float); else PSX_AR(O, M, __nv_bfloat16); } while (0)
     const int opt = s->lay.opt;
-    if (opt == PSX_OPT_SGD && mode == PSX_MODE_SUM) PSX_AR2(PSX_OPT_SGD, PSX_MODE_SUM);
-    else if (opt == PSX_OPT_SGD) PSX_AR2(PSX_OPT_SGD, PSX_MODE_SYNC_MEAN);
-    else if (mode == PSX_MODE_SUM) PSX_AR2(PSX_OPT_ADAM, PSX_MODE_SUM);
-    else PSX_AR2(PSX_OPT_ADAM, PSX_MODE_SYNC_MEAN);
+#define PSX_AR3(O) do { if (mode == PSX_MODE_SUM) PSX_AR2(O, PSX_MODE_SUM); else PSX_AR2(O, PSX_MODE_SYNC_MEAN); } while (0)
+    if (opt == PSX_OPT_SGD) PSX_AR3(PSX_OPT_SGD);
+    else if (opt == PSX_OPT_ADAM) PSX_AR3(PSX_OPT_ADAM);
+    else if (opt == PSX_OPT_MOMENTUM) PSX_AR3(PSX_OPT_MOMENTUM);
+    else if (opt == PSX_OPT_ADAGRAD) PSX_AR3(PSX_OPT_ADAGRAD);
+    else if (opt == PSX_OPT_RMSPROP) PSX_AR3(PSX_OPT_RMSPROP);
+    else return fail(PSX_EINVAL, "unknown optimizer %d", opt);
+#undef PSX_AR3
 #undef PSX_AR2
 #undef PSX_AR
     LAUNCH_CHECK();

@@ -7,7 +7,8 @@
 //   * gradients reduced in registers in a FIXED slot order
 //   * arithmetic spelled with __f*_rn intrinsics: one IEEE-754 rounding per
 //     operation, never contracted to FMA, so results are bit-identical to the
-//     CPU restatement of TF 0.12's ApplyGradientDescent / ApplyAdam
+//     CPU restatements of TF 0.12's ApplyGradientDescent / ApplyAdam /
+//     ApplyMomentum / ApplyAdagrad / ApplyRMSProp
 //   * completion published with a last-CTA ticket + fence.sys + system-scope flag store so the
 //     consumer (another GPU / another process) can wait with a stream memop
 //     instead of a spinning kernel.
@@ -424,6 +425,14 @@ k_list_ldst(const ListChunk *__restrict__ chunks, int n_chunks, char *shard_base
 }
 
 // one thread: take `n` completions off a worker's mailbox (counted rendez-vous)
+// Shard creation: an optimizer state array that does not start at zero.
+__global__ void __launch_bounds__(kCopyThreads) k_fill(float4 *__restrict__ dst, float value, size_t n4)
+{
+    const float4 v = make_float4(value, value, value, value);
+    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += (size_t)gridDim.x * blockDim.x)
+        dst[i] = v;
+}
+
 __global__ void k_consume(unsigned int *counter, unsigned int n) { atomicSub(counter, n); }
 
 // "my gradients for round seq are in place", to up to kMaxSignal shards in ONE
@@ -447,6 +456,15 @@ __global__ void k_signal(SignalSet set, unsigned int seq)
 }
 
 // --------------------------------------------------------------- optimizer ---
+// What each optimizer keeps beside `var`: the number of f32 state arrays (the
+// shard's m, v regions) and whether it carries beta powers advanced once per apply.
+template <int OPT> struct OptTraits;
+template <> struct OptTraits<PSX_OPT_SGD> { static constexpr int kState = 0; static constexpr bool kPowers = false; };
+template <> struct OptTraits<PSX_OPT_ADAM> { static constexpr int kState = 2; static constexpr bool kPowers = true; };
+template <> struct OptTraits<PSX_OPT_MOMENTUM> { static constexpr int kState = 1; static constexpr bool kPowers = false; };
+template <> struct OptTraits<PSX_OPT_ADAGRAD> { static constexpr int kState = 1; static constexpr bool kPowers = false; };
+template <> struct OptTraits<PSX_OPT_RMSPROP> { static constexpr int kState = 2; static constexpr bool kPowers = false; };
+
 // TF 0.12 ApplyGradientDescent: var -= grad * lr           (mnist.py:55)
 __device__ __forceinline__ float sgd1(float var, float g, float lr)
 {
@@ -464,27 +482,61 @@ __device__ __forceinline__ void adam1(float &var, float &m, float &v, float g, f
     var = __fsub_rn(var, __fdiv_rn(num, den));
 }
 
+// TF 0.12 ApplyMomentum (use_nesterov = false): accum = accum * mu + grad; var -= accum * lr
+__device__ __forceinline__ void momentum1(float &var, float &a, float g, float lr, float mu)
+{
+    a = __fadd_rn(__fmul_rn(a, mu), g);
+    var = __fsub_rn(var, __fmul_rn(a, lr));
+}
+
+// TF 0.12 ApplyAdagrad: accum += grad^2; var -= grad * lr * rsqrt(accum), with rsqrt
+// spelled 1 / sqrt (correctly rounded twice) so the GPU and both CPU restatements agree
+__device__ __forceinline__ void adagrad1(float &var, float &a, float g, float lr)
+{
+    a = __fadd_rn(a, __fmul_rn(g, g));
+    var = __fsub_rn(var, __fmul_rn(__fmul_rn(g, lr), __fdiv_rn(1.0f, __fsqrt_rn(a))));
+}
+
+// TF 0.12 ApplyRMSProp (not centered): ms += (grad^2 - ms) * (1 - decay);
+// mom = mom * mu + grad * lr / sqrt(ms + eps); var -= mom
+__device__ __forceinline__ void rmsprop1(float &var, float &ms, float &mom, float g, float lr,
+                                         float omdecay, float mu, float eps)
+{
+    ms = __fadd_rn(ms, __fmul_rn(__fsub_rn(__fmul_rn(g, g), ms), omdecay));
+    mom = __fadd_rn(__fmul_rn(mom, mu), __fdiv_rn(__fmul_rn(g, lr), __fsqrt_rn(__fadd_rn(ms, eps))));
+    var = __fsub_rn(var, mom);
+}
+
 __device__ __forceinline__ float adam_alpha(float lr, float b1p, float b2p)
 {
     float s = __fsqrt_rn(__fsub_rn(1.0f, b2p));
     return __fdiv_rn(__fmul_rn(lr, s), __fsub_rn(1.0f, b1p));
 }
 
+// One element.  The header's hyper-parameters mean, per optimizer:
+//   SGD {lr} | Adam {lr, b1, b2, eps} | Momentum {lr, mu} | Adagrad {lr, init}
+//   RMSProp {lr, decay, mu, eps}
+// omb1 = 1 - b1 and omb2 = 1 - b2, each rounded once; alpha is Adam's step size.
 template <int OPT>
-__device__ __forceinline__ void apply4(float4 &x, float4 &m, float4 &v, const float4 &g,
-                                       float lr, float alpha, float omb1, float omb2, float eps)
+__device__ __forceinline__ void apply1(float &x, float &m, float &v, float g, float lr, float alpha,
+                                       float b1, float b2, float omb1, float omb2, float eps)
 {
-    if (OPT == PSX_OPT_SGD) {
-        x.x = sgd1(x.x, g.x, lr);
-        x.y = sgd1(x.y, g.y, lr);
-        x.z = sgd1(x.z, g.z, lr);
-        x.w = sgd1(x.w, g.w, lr);
-    } else {
-        adam1(x.x, m.x, v.x, g.x, alpha, omb1, omb2, eps);
-        adam1(x.y, m.y, v.y, g.y, alpha, omb1, omb2, eps);
-        adam1(x.z, m.z, v.z, g.z, alpha, omb1, omb2, eps);
-        adam1(x.w, m.w, v.w, g.w, alpha, omb1, omb2, eps);
-    }
+    if (OPT == PSX_OPT_SGD) x = sgd1(x, g, lr);
+    else if (OPT == PSX_OPT_ADAM) adam1(x, m, v, g, alpha, omb1, omb2, eps);
+    else if (OPT == PSX_OPT_MOMENTUM) momentum1(x, m, g, lr, b1);
+    else if (OPT == PSX_OPT_ADAGRAD) adagrad1(x, m, g, lr);
+    else rmsprop1(x, m, v, g, lr, omb1, b2, eps);
+}
+
+template <int OPT>
+__device__ __forceinline__ void apply4(float4 &x, float4 &m, float4 &v, const float4 &g, float lr,
+                                       float alpha, float b1, float b2, float omb1, float omb2,
+                                       float eps)
+{
+    apply1<OPT>(x.x, m.x, v.x, g.x, lr, alpha, b1, b2, omb1, omb2, eps);
+    apply1<OPT>(x.y, m.y, v.y, g.y, lr, alpha, b1, b2, omb1, omb2, eps);
+    apply1<OPT>(x.z, m.z, v.z, g.z, lr, alpha, b1, b2, omb1, omb2, eps);
+    apply1<OPT>(x.w, m.w, v.w, g.w, lr, alpha, b1, b2, omb1, omb2, eps);
 }
 
 __device__ __forceinline__ float4 add4(const float4 &a, const float4 &b)
@@ -510,7 +562,7 @@ __device__ __forceinline__ void finish_apply(ShardHeader *h, const PeerSet &peer
     if (last && threadIdx.x == 0 && !finish) {
         h->ticket = 0;
     } else if (last && threadIdx.x == 0) {
-        if (OPT == PSX_OPT_ADAM) {
+        if (OptTraits<OPT>::kPowers) {
             float p1 = h->b1p, p2 = h->b2p;
             for (int k = 0; k < applies; ++k) {
                 p1 = __fmul_rn(p1, b1);
@@ -615,7 +667,7 @@ __device__ __forceinline__ void finish_served(ShardHeader *h, int count, float b
     h->ticket = 0;
     if (count == 0) return;
     const int applies = (MODE == PSX_MODE_ASYNC_ORDERED) ? count : 1;
-    if (OPT == PSX_OPT_ADAM) {
+    if (OptTraits<OPT>::kPowers) {
         float p1 = h->b1p, p2 = h->b2p;
         for (int k = 0; k < applies; ++k) {
             p1 = __fmul_rn(p1, b1);
@@ -755,7 +807,7 @@ k_apply(ShardHeader *__restrict__ h, float4 *__restrict__ var, float4 *__restric
     const float lr = h->lr, b1 = h->b1, b2 = h->b2, eps = h->eps;
     const float omb1 = __fsub_rn(1.0f, b1);
     const float omb2 = __fsub_rn(1.0f, b2);
-    if (OPT == PSX_OPT_ADAM) {
+    if (OptTraits<OPT>::kPowers) {
         if (threadIdx.x == 0) {
             float p1 = h->b1p, p2 = h->b2p;
             const int na = (MODE == PSX_MODE_ASYNC_ORDERED) ? count : 1;
@@ -787,10 +839,8 @@ k_apply(ShardHeader *__restrict__ h, float4 *__restrict__ var, float4 *__restric
     float4 xn = make_float4(0.f, 0.f, 0.f, 0.f), mn = xn, vn = xn;
     if (i < n4) {
         xn = ld_stream(var + i);
-        if (OPT == PSX_OPT_ADAM) {
-            mn = ld_stream(mom + i);
-            vn = ld_stream(vel + i);
-        }
+        if (OptTraits<OPT>::kState >= 1) mn = ld_stream(mom + i);
+        if (OptTraits<OPT>::kState >= 2) vn = ld_stream(vel + i);
     }
 #endif
     for (; i < n4; i += stride) {
@@ -798,18 +848,14 @@ k_apply(ShardHeader *__restrict__ h, float4 *__restrict__ var, float4 *__restric
         float4 x = xn, m = mn, v = vn;
         if (i + stride < n4) {
             xn = ld_stream(var + i + stride);
-            if (OPT == PSX_OPT_ADAM) {
-                mn = ld_stream(mom + i + stride);
-                vn = ld_stream(vel + i + stride);
-            }
+            if (OptTraits<OPT>::kState >= 1) mn = ld_stream(mom + i + stride);
+            if (OptTraits<OPT>::kState >= 2) vn = ld_stream(vel + i + stride);
         }
 #else
         float4 x = ld_stream(var + i);
         float4 m = make_float4(0.f, 0.f, 0.f, 0.f), v = m;
-        if (OPT == PSX_OPT_ADAM) {
-            m = ld_stream(mom + i);
-            v = ld_stream(vel + i);
-        }
+        if (OptTraits<OPT>::kState >= 1) m = ld_stream(mom + i);
+        if (OptTraits<OPT>::kState >= 2) v = ld_stream(vel + i);
 #endif
         float4 g[kSlotChunk];
         if (PF) {
@@ -837,8 +883,8 @@ k_apply(ShardHeader *__restrict__ h, float4 *__restrict__ var, float4 *__restric
 #pragma unroll
                 for (int k = 0; k < kSlotChunk; ++k)
                     if (s0 + k < count)
-                        apply4<OPT>(x, m, v, g[k], lr, OPT == PSX_OPT_ADAM ? s_alpha[s0 + k] : 0.f,
-                                    omb1, omb2, eps);
+                        apply4<OPT>(x, m, v, g[k], lr, OptTraits<OPT>::kPowers ? s_alpha[s0 + k] : 0.f,
+                                    b1, b2, omb1, omb2, eps);
             } else {
 #pragma unroll
                 for (int k = 0; k < kSlotChunk; ++k)
@@ -847,13 +893,12 @@ k_apply(ShardHeader *__restrict__ h, float4 *__restrict__ var, float4 *__restric
         }
         if (MODE != PSX_MODE_ASYNC_ORDERED) {
             if (MODE == PSX_MODE_SYNC_MEAN) acc = div4(acc, fcount);
-            apply4<OPT>(x, m, v, acc, lr, OPT == PSX_OPT_ADAM ? s_alpha[0] : 0.f, omb1, omb2, eps);
+            apply4<OPT>(x, m, v, acc, lr, OptTraits<OPT>::kPowers ? s_alpha[0] : 0.f, b1, b2, omb1,
+                        omb2, eps);
         }
         st_stream(var + i, x);
-        if (OPT == PSX_OPT_ADAM) {
-            st_stream(mom + i, m);
-            st_stream(vel + i, v);
-        }
+        if (OptTraits<OPT>::kState >= 1) st_stream(mom + i, m);
+        if (OptTraits<OPT>::kState >= 2) st_stream(vel + i, v);
         if (SCATTER) {   // new parameters to every bound worker, cast to the wire dtype (RNE)
             using W = typename WireOf<SRC>::type;
             for (int s = 0; s < peers.n_param; ++s)
@@ -875,7 +920,7 @@ k_apply(ShardHeader *__restrict__ h, float4 *__restrict__ var, float4 *__restric
 //     g  = multimem.ld_reduce.add.v4.f32 [grad_mc + i]   switch fetches the vector from
 //                                                        EVERY worker's gradient buffer
 //                                                        and returns the f32 sum
-//     SGD / Adam on var, m, v in local HBM
+//     the optimizer on var (+ its state arrays) in local HBM
 //     multimem.st.v4.f32 [param_mc + i], var'            switch replicates the store into
 //                                                        EVERY worker's parameter buffer
 // NVLink bytes per GPU and direction for a bucket of B bytes striped over N GPUs:
@@ -899,7 +944,7 @@ k_round_mc(ShardHeader *__restrict__ h, float4 *__restrict__ var, float4 *__rest
     const float lr = h->lr, b1 = h->b1, b2 = h->b2, eps = h->eps;
     const float omb1 = __fsub_rn(1.0f, b1);
     const float omb2 = __fsub_rn(1.0f, b2);
-    const float alpha = (OPT == PSX_OPT_ADAM) ? adam_alpha(lr, h->b1p, h->b2p) : 0.f;
+    const float alpha = OptTraits<OPT>::kPowers ? adam_alpha(lr, h->b1p, h->b2p) : 0.f;
     const float fdiv = (float)divisor;
 
     const size_t tile = (size_t)kMcThreads * U;
@@ -921,10 +966,8 @@ k_round_mc(ShardHeader *__restrict__ h, float4 *__restrict__ var, float4 *__rest
             const size_t i = base + (size_t)u * kMcThreads;
             if (i < n4) {
                 x[u] = ld_stream(var + i);
-                if (OPT == PSX_OPT_ADAM) {
-                    m[u] = ld_stream(mom + i);
-                    v[u] = ld_stream(vel + i);
-                }
+                if (OptTraits<OPT>::kState >= 1) m[u] = ld_stream(mom + i);
+                if (OptTraits<OPT>::kState >= 2) v[u] = ld_stream(vel + i);
             }
         }
 #pragma unroll
@@ -943,12 +986,10 @@ k_round_mc(ShardHeader *__restrict__ h, float4 *__restrict__ var, float4 *__rest
             if (i < n4) {
                 float4 acc = g[u];
                 if (MODE == PSX_MODE_SYNC_MEAN) acc = div4(acc, fdiv);
-                apply4<OPT>(x[u], m[u], v[u], acc, lr, alpha, omb1, omb2, eps);
+                apply4<OPT>(x[u], m[u], v[u], acc, lr, alpha, b1, b2, omb1, omb2, eps);
                 st_stream(var + i, x[u]);
-                if (OPT == PSX_OPT_ADAM) {
-                    st_stream(mom + i, m[u]);
-                    st_stream(vel + i, v[u]);
-                }
+                if (OptTraits<OPT>::kState >= 1) st_stream(mom + i, m[u]);
+                if (OptTraits<OPT>::kState >= 2) st_stream(vel + i, v[u]);
                 mc_st(param_mc + 4 * i, x[u]);
             }
         }
@@ -1011,8 +1052,8 @@ __device__ __forceinline__ long long rows_find(const long long *idx, long long n
 // One warp per pushed entry (slot w, position k).  The entry whose worker is the
 // LOWEST one holding that row index is the row's representative: it sums the
 // row's contributions in worker order ((g_w + g_w') + ...), divides for MEAN, and
-// applies SGD / Adam to that row of var (m, v) only -- untouched rows keep their
-// value and their moments ("lazy" sparse semantics).
+// applies the optimizer to that row of var (m, v) only -- untouched rows keep their
+// value and their state ("lazy" sparse semantics, TF's SparseApply*).
 template <int OPT, int MODE, typename WIRE>
 __global__ void __launch_bounds__(256)
 k_apply_rows(ShardHeader *__restrict__ h, float *__restrict__ var, float *__restrict__ mom,
@@ -1021,7 +1062,7 @@ k_apply_rows(ShardHeader *__restrict__ h, float *__restrict__ var, float *__rest
 {
     const float lr = h->lr, b1 = h->b1, b2 = h->b2, eps = h->eps;
     const float omb1 = __fsub_rn(1.0f, b1), omb2 = __fsub_rn(1.0f, b2);
-    const float alpha = (OPT == PSX_OPT_ADAM) ? adam_alpha(lr, h->b1p, h->b2p) : 0.f;
+    const float alpha = OptTraits<OPT>::kPowers ? adam_alpha(lr, h->b1p, h->b2p) : 0.f;
     const float fcount = (float)count;
     const int lane = threadIdx.x & 31;
     const size_t warp = ((size_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
@@ -1067,15 +1108,12 @@ k_apply_rows(ShardHeader *__restrict__ h, float *__restrict__ var, float *__rest
             }
             if (MODE == PSX_MODE_SYNC_MEAN) g = __fdiv_rn(g, fcount);
             const size_t at = (size_t)row * d + j;
-            float x = var[at];
-            if (OPT == PSX_OPT_SGD) {
-                x = sgd1(x, g, lr);
-            } else {
-                float m = mom[at], v = vel[at];
-                adam1(x, m, v, g, alpha, omb1, omb2, eps);
-                mom[at] = m;
-                vel[at] = v;
-            }
+            float x = var[at], m = 0.f, v = 0.f;
+            if (OptTraits<OPT>::kState >= 1) m = mom[at];
+            if (OptTraits<OPT>::kState >= 2) v = vel[at];
+            apply1<OPT>(x, m, v, g, lr, alpha, b1, b2, omb1, omb2, eps);
+            if (OptTraits<OPT>::kState >= 1) mom[at] = m;
+            if (OptTraits<OPT>::kState >= 2) vel[at] = v;
             var[at] = x;
         }
     }

@@ -4,6 +4,8 @@ replication that the reference's examples use, re-expressed over libpsx.so.
     replica_device_setter      examples/mnist/mnist.py:43, mnist_replica.py:116
     GradientDescentOptimizer   mnist.py:55, matrix_factorization.py:39
     AdamOptimizer              mnist_replica.py:147
+    MomentumOptimizer, AdagradOptimizer, RMSPropOptimizer
+                               TF 0.12's tf.train classes of the same names
     ParameterServer            the process behind tf.train.Server for job 'ps'
                                (tfmesos/server.py:51-66, mnist_replica.py:93-95)
     Worker                     the session a worker opens on the PS devices
@@ -25,12 +27,17 @@ STRIPE_ALIGN = 1024  # stripes start on 4 KiB boundaries
 
 
 class GradientDescentOptimizer(object):
-    """tf.train.GradientDescentOptimizer(learning_rate) (mnist.py:55)."""
+    """tf.train.GradientDescentOptimizer(learning_rate) (mnist.py:55).
+
+    Every optimizer class carries ``opt`` (the PSX_OPT_* id) and ``hyper``, the
+    four floats the shard header holds (include/psx.h lists their meaning)."""
     opt = psx.OPT_SGD
 
     def __init__(self, learning_rate):
         self.learning_rate = float(learning_rate)
-        self.beta1, self.beta2, self.epsilon = 0.9, 0.999, 1e-8
+        # the unused slots keep Adam's defaults: the header's stored powers, and so
+        # the checkpoint metadata, stay what they have always been for SGD
+        self.hyper = (self.learning_rate, 0.9, 0.999, 1e-8)
 
 
 class AdamOptimizer(object):
@@ -40,6 +47,45 @@ class AdamOptimizer(object):
     def __init__(self, learning_rate=0.001, beta1=0.9, beta2=0.999, epsilon=1e-8):
         self.learning_rate = float(learning_rate)
         self.beta1, self.beta2, self.epsilon = float(beta1), float(beta2), float(epsilon)
+        self.hyper = (self.learning_rate, self.beta1, self.beta2, self.epsilon)
+
+
+class MomentumOptimizer(object):
+    """tf.train.MomentumOptimizer(learning_rate, momentum) (use_nesterov=False):
+    accum = accum * momentum + grad; var -= accum * lr.  accum starts at 0."""
+    opt = psx.OPT_MOMENTUM
+
+    def __init__(self, learning_rate, momentum):
+        self.learning_rate, self.momentum = float(learning_rate), float(momentum)
+        self.hyper = (self.learning_rate, self.momentum, 0.0, 0.0)
+
+
+class AdagradOptimizer(object):
+    """tf.train.AdagradOptimizer(learning_rate, initial_accumulator_value=0.1):
+    accum += grad^2; var -= grad * lr / sqrt(accum).  accum starts at
+    initial_accumulator_value, which must be positive."""
+    opt = psx.OPT_ADAGRAD
+
+    def __init__(self, learning_rate, initial_accumulator_value=0.1):
+        if not initial_accumulator_value > 0.0:
+            raise ValueError("initial_accumulator_value must be positive: %r"
+                             % (initial_accumulator_value,))
+        self.learning_rate = float(learning_rate)
+        self.initial_accumulator_value = float(initial_accumulator_value)
+        self.hyper = (self.learning_rate, self.initial_accumulator_value, 0.0, 0.0)
+
+
+class RMSPropOptimizer(object):
+    """tf.train.RMSPropOptimizer(learning_rate, decay=0.9, momentum=0.0,
+    epsilon=1e-10) (centered=False): ms += (grad^2 - ms) * (1 - decay);
+    mom = mom * momentum + grad * lr / sqrt(ms + epsilon); var -= mom.
+    ms starts at 1 (TF's ``rms`` slot), mom at 0."""
+    opt = psx.OPT_RMSPROP
+
+    def __init__(self, learning_rate, decay=0.9, momentum=0.0, epsilon=1e-10):
+        self.learning_rate = float(learning_rate)
+        self.decay, self.momentum, self.epsilon = float(decay), float(momentum), float(epsilon)
+        self.hyper = (self.learning_rate, self.decay, self.momentum, self.epsilon)
 
 
 def replica_device_setter(ps_tasks=0, cluster=None):
@@ -157,9 +203,7 @@ class ParameterServer(object):
         self.spec = spec
         self.n_workers = int(n_workers)
         self.device = spec.device if device is None else int(device)
-        self.shard = psx.Shard(self.device, spec.nelem, optimizer.opt,
-                               optimizer.learning_rate, optimizer.beta1, optimizer.beta2,
-                               optimizer.epsilon,
+        self.shard = psx.Shard(self.device, spec.nelem, optimizer.opt, *optimizer.hyper,
                                n_slots=self.n_workers if landing_slots else 0, wire=wire)
 
     def handle(self):

@@ -13,8 +13,10 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 # TFMESOS_PSX_LIB selects another build of the same ABI (kernel A/B experiments)
 LIB_PATH = os.environ.get("TFMESOS_PSX_LIB") or os.path.join(HERE, "lib", "libpsx.so")
 
-ABI_VERSION = 10
-OPT_SGD, OPT_ADAM = 0, 1
+ABI_VERSION = 11
+OPT_SGD, OPT_ADAM, OPT_MOMENTUM, OPT_ADAGRAD, OPT_RMSPROP = 0, 1, 2, 3, 4
+# f32 state arrays each optimizer keeps beside var: PSX_M [, PSX_V]
+OPT_STATE_ARRAYS = {OPT_SGD: 0, OPT_ADAM: 2, OPT_MOMENTUM: 1, OPT_ADAGRAD: 1, OPT_RMSPROP: 2}
 MODE_ASYNC_ORDERED, MODE_SUM, MODE_SYNC_MEAN = 0, 1, 2
 F32, BF16 = 0, 1
 VAR, M, V, SLOT0 = 0, 1, 2, 16

@@ -18,8 +18,8 @@ from contextlib import contextmanager
 
 from . import endpoint, engine, psx
 from .utils import bind_advertised
-from .engine import (AdamOptimizer, GradientDescentOptimizer,  # noqa: F401
-                     replica_device_setter)
+from .engine import (AdagradOptimizer, AdamOptimizer, GradientDescentOptimizer,  # noqa: F401
+                     MomentumOptimizer, RMSPropOptimizer, replica_device_setter)
 
 
 class ClusterSpec(object):
@@ -130,7 +130,7 @@ class ParameterClient(object):
         # the shard by handle; the topology only records one stripe per task
         self.topo = engine.Topology(self.layout, ps_devices,
                                     [device] * self.n_workers)
-        hyper = (optimizer.learning_rate, optimizer.beta1, optimizer.beta2, optimizer.epsilon)
+        hyper = optimizer.hyper
         handles = {}
         for spec in self.topo.shards:
             handles[spec.key] = endpoint.call(
